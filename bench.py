@@ -10,7 +10,7 @@ fixed model): the ranks form a pipeline -- every step a rank receives the hidden
 from rank - 1 and sends its own to rank + 1 (NCCL point-to-point over NVLink, overlapped with the kernels) -- and
 the only collective is ONE all-reduce(MAX) of the amax arena per calibration job (the timed K steps are one job).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Prints one JSON line (rank 0).  See DESIGN.md "Measurement" for every key.
 """
@@ -492,13 +492,21 @@ def run_gpu(args):
 
     eng = ShardedPTQEngine(plan, TOKENS, "nvfp4", torch.bfloat16, dev, rank, world, allreduce_every=args.steps)
     acts = eng.alloc_activations(seed=0)
-    outs = eng.alloc_outputs(4)
+    # fake-quant outputs: a ring of four buffers (quantizer i writes slot i % 4), except the last four quantizers,
+    # which get buffers of their own.  In the ring, several quantizers of one grouped launch write the same slot, so
+    # what a slot holds afterwards depends on the order in which CTAs run; the own buffers hold exactly those four
+    # quantizers' outputs after a step (--dump-outputs reads them).  Same bytes written either way.
+    ring = eng.alloc_outputs(4)
+    nq = len(eng.quantizers)
+    outs = [ring[i % 4] for i in range(nq - 4)] + [torch.empty(x.numel(), dtype=x.dtype, device=dev) for x in acts[nq - 4:]]
     eng.capture(acts, outs)
 
     # ---- device-resident timing (value) -------------------------------------------------------------
     sampler = ClockSampler(local) if rank == 0 else None
     ms_step, (t_wall0, t_wall1) = timed_job(eng, args.steps, max(args.warmup, 3), sampler)
     clocks = sampler.stop(t_wall0, t_wall1) if rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(eng, acts, outs, args.dump_outputs, rank, world)
     value = TOKENS / (ms_step * 1e-3)
     comm_counts = dict(eng.comm_log)
 
@@ -649,6 +657,37 @@ def run_gpu(args):
         dist.destroy_process_group()
 
 
+DUMP_ROWS = 256           # token rows of each dumped activation, shared out over the ranks
+DUMP_BUDGET = 64 << 20    # bytes --dump-outputs may write over all ranks
+
+
+def dump_outputs(eng, acts, outs, out_dir, rank, world):
+    """Write what the last timed step left on the device as ``out_dir/<name>.npy`` (float32): the fp32 amax arena
+    (``amax``), the amax exported to the quantizers (``amax_export``) and the fake-quantized activations of the last
+    four quantizers, which have output buffers of their own (``fake_quant.<quantizer>``), on DUMP_ROWS // world token
+    rows drawn with a fixed seed.  With several GPUs every name is prefixed by ``rank<r>.``.  The rows are split over
+    the ranks so that the total stays bounded: at most 256 x (3 x 8192 + 28672) x 4 B = 54.5 MB of activations over all
+    ranks (Llama-3-70B; 27.3 MB for Llama-3-8B), plus 8 B per quantizer of amax per rank."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    prefix = f"rank{rank}." if world > 1 else ""
+    n_rows = max(1, DUMP_ROWS // world)
+    rows = torch.randperm(TOKENS, generator=torch.Generator().manual_seed(0))[:n_rows].sort().values
+    arrays = {"amax": eng.global_arena, "amax_export": eng.amax_arena}
+    parity = (eng._step - 1) & 1 if eng.handoff else 0
+    last_hidden = len(eng.quantizers) - 4 if (eng.handoff and eng.hand_out is not None) else -1
+    for i in range(len(eng.quantizers) - 4, len(eng.quantizers)):
+        x = acts[i]
+        y = eng.hand_out[parity] if i == last_hidden else outs[i % len(outs)][: x.numel()].view_as(x)
+        arrays[f"fake_quant.{eng.quantizers[i][0]}"] = y[rows.to(y.device)]
+    nbytes = sum(t.numel() * 4 for t in arrays.values())
+    assert nbytes * world <= DUMP_BUDGET, f"--dump-outputs would write {nbytes * world} bytes over {world} ranks"
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), t.float().cpu().numpy())
+
+
 def run_e2e(eng, acts, outs, dev, world, args, barrier):
     """Same step through the engine API with HOST buffers: every step copies each quantizer's
     activation from pinned host memory into its device buffer (copy stream, overlapped with the collect
@@ -720,7 +759,14 @@ def main():
                          "(32 = full model, 0 = skip; N=1 only; a context number, not the headline)")
     ap.add_argument("--model", default="llama-3-8b", choices=["llama-3-8b", "llama-3-70b"],
                     help="shape plan; the default is the BASELINE metric's model (70b = BASELINE config 5)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float32, same seeded inputs on "
+                         "every run) so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's outputs; it does not apply to --impl reference")
     if args.impl == "reference":
         run_reference(args)
     else:

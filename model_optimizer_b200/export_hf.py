@@ -14,7 +14,7 @@ layout) and the formats this engine packs (FP8, NVFP4 dynamic / static, INT4-AWQ
     renamed to ``pre_quant_scale``;
   * ``hf_quant_config.json`` (quant_utils.py:1583-1700, convert_hf_quant_config_format) and ``model.safetensors``.
 
-Pinned byte for byte against the reference's own export of the same calibrated state (tests/golden/ref_export.npz).
+Pinned byte for byte against the reference's own export of the same calibrated state (tests/golden/ref_export.*.npz).
 """
 
 from __future__ import annotations

@@ -18,6 +18,8 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 OUT = os.path.join(ROOT, "tests", "golden")
+sys.path.insert(0, os.path.join(ROOT, "tests"))
+import _golden  # noqa: E402  (the fixtures' file format: split into parts under 1 MB)
 
 
 def _install_shim():
@@ -191,8 +193,7 @@ def main():
                 out[f"{key}/hist2_edges_last"] = hc._calib_bin_edges[-1].numpy().copy()
 
     out["cases"] = np.array(cases)
-    np.savez_compressed(os.path.join(OUT, "ref_small.npz"), **out)
-    print("wrote", os.path.join(OUT, "ref_small.npz"), len(out), "arrays")
+    print("wrote", _golden.save("ref_small", out, OUT), len(out), "arrays")
 
 
 
@@ -427,8 +428,7 @@ def main_mx():
         out[f"qt/{dname}/ragged/mxfp8/q"] = q8._quantized_data.view(torch.uint8).numpy().copy()
         out[f"qt/{dname}/ragged/mxfp8/scale"] = s8.numpy().copy()
         out[f"qt/{dname}/ragged/mxfp8/deq"] = q8.dequantize(dtype=dt, scale=s8).float().numpy().view(np.uint32)
-    np.savez_compressed(os.path.join(OUT, "ref_mx.npz"), **out)
-    print("wrote", os.path.join(OUT, "ref_mx.npz"), len(out), "arrays")
+    print("wrote", _golden.save("ref_mx", out, OUT), len(out), "arrays")
 
 
 def main_bias():
@@ -511,8 +511,7 @@ def main_fp8_blocks():
                 wsf = (tq.amax.float() / 448.0).squeeze()
                 q2, _ = FP8QTensor.quantize(x, wsf, block_sizes=dict(blocks))
                 out[key + "/q_export"] = q2._quantized_data.view(torch.uint8).numpy().copy()
-    np.savez_compressed(os.path.join(OUT, "ref_fp8_blocks.npz"), **out)
-    print("wrote", os.path.join(OUT, "ref_fp8_blocks.npz"), len(out), "arrays")
+    print("wrote", _golden.save("ref_fp8_blocks", out, OUT), len(out), "arrays")
 
 
 def main_int8():
@@ -702,7 +701,7 @@ def main_export():
                re-calibrating on different hardware;
       out/...  every tensor of the exported ``model.safetensors`` as raw bytes + dtype + shape;
       cfg      ``hf_quant_config.json``.
-    -> tests/golden/ref_export.npz"""
+    -> tests/golden/ref_export.*.npz"""
     _install_shim()
     import copy
     import json
@@ -758,8 +757,7 @@ def main_export():
                 out[f"{key}/meta/{k}"] = np.array(json.dumps([str(v.dtype), list(v.shape)]))
             out[f"{key}/cfg"] = np.array(json.dumps(json.load(open(os.path.join(d, "hf_quant_config.json")))))
         print("export", key, len(sd), "tensors", json.loads(str(out[f"{key}/cfg"]))["quantization"])
-    np.savez_compressed(os.path.join(OUT, "ref_export.npz"), **out)
-    print("wrote ref_export.npz", len(out), "arrays", os.path.getsize(os.path.join(OUT, "ref_export.npz")) >> 10, "KiB")
+    print("wrote", _golden.save("ref_export", out, OUT), len(out), "arrays")
 
 
 if __name__ == "__main__":

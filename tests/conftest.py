@@ -14,6 +14,6 @@ def pytest_configure(config):
 
 @pytest.fixture(scope="session")
 def golden():
-    import numpy as np
+    import _golden
 
-    return np.load(os.path.join(ROOT, "tests", "golden", "ref_small.npz"))
+    return _golden.load("ref_small")

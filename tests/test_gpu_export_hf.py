@@ -1,11 +1,12 @@
 """Unified-HF export (SURVEY.md 8(f1)) byte for byte against the reference's ``export_hf_checkpoint`` of the SAME
-calibrated state (tests/golden/ref_export.npz, made by oracle/gen_golden.py export with the real reference on CPU):
+calibrated state (tests/golden/ref_export.*.npz, made by oracle/gen_golden.py export with the real reference on CPU):
 FP8, NVFP4 (dynamic and static weights) and INT4-AWQ (re-smoothing of q/k/v and gate/up to one averaged
 pre_quant_scale, folded into the preceding norm)."""
 
 import json
 import os
 
+import _golden
 import numpy as np
 import pytest
 import torch
@@ -18,7 +19,7 @@ TD = {"torch.bfloat16": torch.bfloat16, "torch.float32": torch.float32, "torch.f
 
 @pytest.fixture(scope="module")
 def fx():
-    return np.load(os.path.join(ROOT, "tests", "golden", "ref_export.npz"))
+    return _golden.load("ref_export")
 
 
 def build_calibrated(fx, key, preset):

@@ -1,10 +1,11 @@
 """GPU parity of the MX (E8M0 block scale) kernels, called through the C-ABI, against
-(a) tests/golden/ref_mx.npz -- outputs of the reference's own C++ (host builds of tensor_quant_mx.h/.cu)
+(a) tests/golden/ref_mx.*.npz -- outputs of the reference's own C++ (host builds of tensor_quant_mx.h/.cu)
     and of its MXFP8 / MXFP4 QTensor Python, and
 (b) the NumPy oracle on larger / irregular tensors.  Bar: bit-exact."""
 
 import os
 
+import _golden
 import numpy as np
 import pytest
 import torch
@@ -14,7 +15,7 @@ from oracle import oracle_np as o
 pytestmark = pytest.mark.gpu
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-G = np.load(os.path.join(ROOT, "tests", "golden", "ref_mx.npz"))
+G = _golden.load("ref_mx")
 TD = {"bf16": torch.bfloat16, "f16": torch.float16, "f32": torch.float32}
 FMT_NAMES = ["E4M3", "E5M2", "INT8", "E0M3", "E1M2", "E3M0", "E2M1", "E3M2", "E2M3"]
 

@@ -4,6 +4,7 @@ quantize()) against the oracle and the whole-algorithm reference fixtures."""
 import copy
 import os
 
+import _golden
 import numpy as np
 import pytest
 import torch
@@ -588,7 +589,7 @@ def test_bias_calibrator_and_affine_quantizer():
 def test_fp8_block_scales_eager_rule_and_2d_blocks(ops):
     """FP8 with static 1-D / 2-D block scales (FP8_2D_BLOCKWISE_WEIGHT_ONLY_CFG): the quantizer's tile amax, the
     eager-rule fake quant the reference runs for multi-dim amax (tensor_quant.py:78-79), FP8QTensor pack / dequant
-    with block_sizes and the fp8_pb_wo export -- against the reference run on CPU (tests/golden/ref_fp8_blocks.npz)."""
+    with block_sizes and the fp8_pb_wo export -- against the reference run on CPU (tests/golden/ref_fp8_blocks.*.npz)."""
     import os
 
     import model_optimizer_b200.config as cfgs
@@ -597,7 +598,7 @@ def test_fp8_block_scales_eager_rule_and_2d_blocks(ops):
     from model_optimizer_b200.nn import TensorQuantizer
     from model_optimizer_b200.qtensor import FP8QTensor
 
-    G = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_fp8_blocks.npz"))
+    G = _golden.load("ref_fp8_blocks")
     keys = sorted({k.rsplit("/x", 1)[0] for k in G.files if k.endswith("/x")})
     assert len(keys) == 12
     for key in keys:

@@ -10,7 +10,9 @@ Triton divides with `div.full.f32` (2-ulp approximate); this engine restates the
 They can therefore differ exactly where a quotient sits within an ulp or two of a rounding boundary -- for
 16-bit data that includes the many EXACT real-arithmetic ties (see test_gpu_vs_reference_ext.py), for fp32
 data it is a handful of elements.  The tests bound and report those rates; everything else must be equal.
-Skipped when the cubins are absent."""
+Where the cubins are absent the reference side is what they produced on the same inputs, stored in
+tests/golden/ref_gpu_triton/ (see tests/_refgold.py), and the mismatches in the stored rows count against the bound
+for the whole tensor; only the speed comparison needs the cubins and is skipped then."""
 
 import ctypes
 import json
@@ -19,6 +21,7 @@ import os
 import numpy as np
 import pytest
 import torch
+from _refgold import RefResults, Store
 
 from oracle import oracle_np as o
 
@@ -28,6 +31,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REF = os.path.join(ROOT, "oracle", "_ref")
 DN = {torch.bfloat16: "bf16", torch.float16: "f16", torch.float32: "f32"}
 REPORT = {}
+LIVE = os.path.exists(os.path.join(REF, "triton_kernels.json")) and os.path.exists(
+    os.path.join(REF, "modelopt_cuda_ext_fp8.so"))
 
 
 class RefTritonKernel:
@@ -63,6 +68,18 @@ class RefTritonKernel:
 
 
 @pytest.fixture(scope="module")
+def store():
+    s = Store("ref_gpu_triton", LIVE)
+    yield s
+    s.save()
+
+
+@pytest.fixture
+def refs(store, request):
+    return RefResults(store, request.node.name)
+
+
+@pytest.fixture(scope="module")
 def ops():
     from model_optimizer_b200 import ops as _ops
 
@@ -79,16 +96,20 @@ def inputs(shape, dtype, seed, kind="gauss"):
     return x.to(dtype)
 
 
+def ref_global_scale(global_amax):
+    return global_amax.float() / (6.0 * 448.0)        # :140, evaluated by torch on the GPU like the reference
+
+
 def ref_fp4_fake_quant_block(x, global_amax):
     """fp4_fake_quant_block (fp4_kernel_hopper.py:102-170) with the compiled reference kernel."""
     k = RefTritonKernel(f"fp4_fake_quant_{DN[x.dtype]}")
     x2 = x.reshape(-1, x.shape[-1]).contiguous()
     y = torch.empty_like(x2)
     m, n = x2.shape
-    gs = (global_amax.float() / (6.0 * 448.0)).to(x.device)        # :140, evaluated by torch on the GPU like the reference
+    gs = ref_global_scale(global_amax).to(x.device)
     k(((m + 15) // 16, (n + 63) // 64), x2.data_ptr(), y.data_ptr(), m, n, gs.data_ptr(), x2.stride(0), x2.stride(1),
       y.stride(0), y.stride(1))
-    return y.view(x.shape), gs
+    return y.view(x.shape)
 
 
 def mismatch_stats(ref, got):
@@ -102,16 +123,17 @@ def mismatch_stats(ref, got):
 
 
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16, torch.float16])
-def test_nvfp4_dynamic_vs_reference_triton(ops, dtype):
+def test_nvfp4_dynamic_vs_reference_triton(ops, refs, dtype):
     rep = {}
     for kind, shape in (("gauss", (1024, 4096)), ("heavy", (1024, 4096)), ("scaled", (512, 4096)), ("ragged", (300, 200))):
         x = inputs(shape, dtype, 11, "gauss" if kind == "ragged" else kind)
         g = x.abs().max().float().reshape(1)
-        ref, gs = ref_fp4_fake_quant_block(x, g)
         got = ops.fake_quant_nvfp4(x, g)
+        ref, got = refs.rows(got, lambda: ref_fp4_fake_quant_block(x, g))
+        gs = ref_global_scale(g)
         gs_ieee = g / torch.tensor(6.0 * 448.0, device="cuda")
         n, bounded = mismatch_stats(ref, got)
-        rep[kind] = {"elements": x.numel(), "mismatches": n, "rate": n / x.numel(),
+        rep[kind] = {"elements": x.numel(), "compared": ref.numel(), "mismatches": n, "rate": n / ref.numel(),
                      "global_scale_same_as_ieee": bool(torch.equal(gs, gs_ieee))}
         assert bounded, (dtype, kind)
         if torch.equal(gs, gs_ieee):
@@ -122,50 +144,60 @@ def test_nvfp4_dynamic_vs_reference_triton(ops, dtype):
 
 
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
-def test_nvfp4_static_vs_reference_triton(ops, dtype):
+def test_nvfp4_static_vs_reference_triton(ops, refs, dtype):
     """static_blockwise_fp4_fake_quant (fp4_kernel.py:253-316): scales from compute_fp4_scales evaluated the way
     the reference does on the GPU (torch ops + its own FP8 extension), then its Triton kernel."""
     import importlib.machinery
     import importlib.util
 
-    p = os.path.join(REF, "modelopt_cuda_ext_fp8.so")
-    if not os.path.exists(p):
-        pytest.skip("reference fp8 extension not built")
-    loader = importlib.machinery.ExtensionFileLoader("modelopt_cuda_ext_fp8", p)
-    ext8 = importlib.util.module_from_spec(importlib.util.spec_from_loader("modelopt_cuda_ext_fp8", loader))
-    loader.exec_module(ext8)
-    k = RefTritonKernel(f"fp4_static_{DN[dtype]}")
-    rep = {}
-    for kind in ("gauss", "heavy", "scaled"):
-        x = inputs((1024, 2048), dtype, 12, kind)
-        amax = x.view(-1, 16).abs().amax(dim=-1).float()
-        g = amax.max()
+    def reference(x, amax, g):
+        p = os.path.join(REF, "modelopt_cuda_ext_fp8.so")
+        if not os.path.exists(p):
+            pytest.skip("reference fp8 extension not built")
+        loader = importlib.machinery.ExtensionFileLoader("modelopt_cuda_ext_fp8", p)
+        ext8 = importlib.util.module_from_spec(importlib.util.spec_from_loader("modelopt_cuda_ext_fp8", loader))
+        loader.exec_module(ext8)
+        k = RefTritonKernel(f"fp4_static_{DN[dtype]}")
         scale = amax / 6.0                                                     # :232
         scale = ext8.fake_e4m3fy(scale, (g * (448.0 / 448.0) / 6.0).reshape(1))   # :243-244 -> scaled_e4m3_impl
         xf = x.contiguous().view(-1)
         y = torch.empty_like(xf)
         k((amax.numel(),), xf.data_ptr(), y.data_ptr(), scale.contiguous().data_ptr(), amax.numel())
+        return y.view(x.shape)
+
+    rep = {}
+    for kind in ("gauss", "heavy", "scaled"):
+        x = inputs((1024, 2048), dtype, 12, kind)
+        amax = x.view(-1, 16).abs().amax(dim=-1).float()
+        g = amax.max()
         got = ops.fake_quant_nvfp4_static(x, amax, g.reshape(1), True, 448.0)
-        n, bounded = mismatch_stats(y.view(x.shape), got)
-        rep[kind] = {"elements": x.numel(), "mismatches": n, "rate": n / x.numel()}
+        ref, got = refs.rows(got, lambda: reference(x, amax, g))
+        n, bounded = mismatch_stats(ref, got)
+        rep[kind] = {"elements": x.numel(), "compared": ref.numel(), "mismatches": n, "rate": n / ref.numel()}
         assert bounded, (dtype, kind)
         assert n <= (1e-3 if dtype == torch.float32 else 0.02) * x.numel(), (dtype, kind, n)
     REPORT[f"nvfp4_static_{DN[dtype]}"] = rep
 
 
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
-def test_fp8_scale_sweep_vs_reference_triton(ops, dtype):
+def test_fp8_scale_sweep_vs_reference_triton(ops, refs, dtype):
     """nvfp4_fp8_scale_sweep (nvfp4_fp8_sweep.py:127-160).  The winner is an argmin over 126 fp32 losses; the two
     implementations sum 16 squared errors in a different order and divide differently, so near-equal losses can
     swap: report the agreement rate."""
-    k = RefTritonKernel(f"fp8_sweep_{DN[dtype]}")
     w = inputs((1024, 1024), dtype, 13, "gauss")
     g = w.abs().max().float().reshape(1)
-    cand = torch.from_numpy(o.fp8_scale_candidates().astype(np.float32)).cuda()
     n_blocks = w.numel() // 16
-    best = torch.empty(n_blocks, dtype=torch.float32, device="cuda")
-    k(((n_blocks + 63) // 64,), w.contiguous().data_ptr(), cand.data_ptr(), g.data_ptr(), best.data_ptr(), n_blocks)
+
+    def reference():
+        k = RefTritonKernel(f"fp8_sweep_{DN[dtype]}")
+        cand = torch.from_numpy(o.fp8_scale_candidates().astype(np.float32)).cuda()
+        best = torch.empty(n_blocks, dtype=torch.float32, device="cuda")
+        k(((n_blocks + 63) // 64,), w.contiguous().data_ptr(), cand.data_ptr(), g.data_ptr(), best.data_ptr(), n_blocks)
+        return best
+
     got = ops.nvfp4_fp8_scale_sweep(w, g, candidates="ieee").reshape(-1)      # the cubin is fed the same IEEE candidates
+    best, _ = refs.rows(got, reference)                                         # all blocks: small enough to store whole
+    best = best.reshape(-1)
     same = float((best == got).float().mean())
     REPORT[f"fp8_sweep_{DN[dtype]}"] = {"blocks": n_blocks, "same_winner": same}
     assert same >= 0.97, same

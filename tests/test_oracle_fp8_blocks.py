@@ -1,17 +1,18 @@
 """FP8 with static 2-D / 1-D block scales: the oracle (eager-rule FP8 fake quant and FP8 pack, applied through the
 [A, b1, B, b2] tile view with the tile amax spread over rows) vs the reference run on CPU
-(tests/golden/ref_fp8_blocks.npz, written by oracle/gen_golden.py fp8_blocks)."""
+(tests/golden/ref_fp8_blocks.*.npz, written by oracle/gen_golden.py fp8_blocks)."""
 
 import os
 import sys
 
+import _golden
 import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
 import oracle_np as o  # noqa: E402
 
-G = np.load(os.path.join(ROOT, "tests", "golden", "ref_fp8_blocks.npz"))
+G = _golden.load("ref_fp8_blocks")
 F32 = np.float32
 
 

@@ -1,5 +1,5 @@
 """The oracle (oracle/oracle_np.py) must reproduce, bit for bit, what the REAL reference produced
-in this container (tests/golden/ref_small.npz, written by oracle/gen_golden.py) and the
+in this container (tests/golden/ref_small.*.npz, written by oracle/gen_golden.py) and the
 reference's own known-answer vectors.  CPU only."""
 
 import numpy as np

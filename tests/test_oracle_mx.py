@@ -1,10 +1,13 @@
 """The NumPy oracle's MX section must reproduce, bit for bit, what the REAL reference produced:
 its C++ element rounding / E8M0 block math (host builds of tensor_quant_mx.h / .cu, oracle/_ref) and
-its MXFP8 / MXFP4 QTensor round trips (tests/golden/ref_mx.npz, written by oracle/gen_golden.py mx)."""
+its MXFP8 / MXFP4 QTensor round trips (tests/golden/ref_mx.*.npz, written by oracle/gen_golden.py mx)."""
 
+import hashlib
+import json
 import os
 import sys
 
+import _golden
 import numpy as np
 import pytest
 
@@ -12,7 +15,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
 import oracle_np as o  # noqa: E402
 
-G = np.load(os.path.join(ROOT, "tests", "golden", "ref_mx.npz"))
+G = _golden.load("ref_mx")
 F32 = np.float32
 
 
@@ -71,18 +74,36 @@ def test_mxfp4_qtensor(dname, kind, bs):
     assert same(o.unpack_mxfp4(packed, scale, bs, dtype=dname), f(G[key + f"/mxfp4_{bs}/deq"])).all()
 
 
+def _digest(a):
+    a = np.asarray(a, F32)
+    return hashlib.sha256(np.where(np.isnan(a), F32(np.nan), a).astype(F32).tobytes()).hexdigest()
+
+
 def test_ref_libs_live():
-    """Where oracle/_ref was built (this container), re-check the restatement against the live libraries."""
+    """The restatement against the reference's element rounding (host build of tensor_quant_mx.h) on a larger random
+    set: live where oracle/_ref was built, else against the SHA-256 of what that build returned
+    (tests/golden/ref_mx_cvt_sha256.json; NaN payloads made equal).  B200Q_RECORD_GOLDEN=<dir> on a live run writes
+    that file to <dir>."""
     import ctypes
 
     p = os.path.join(ROOT, "oracle", "_ref", "libmxref.so")
-    if not os.path.exists(p):
-        pytest.skip("oracle/_ref not built here")
-    h = ctypes.CDLL(p)
-    h.ref_convert_to_exmy_n.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_long, ctypes.c_int]
+    stored = os.path.join(ROOT, "tests", "golden", "ref_mx_cvt_sha256.json")
     rng = np.random.default_rng(5)
     x = np.concatenate([rng.standard_normal(20000).astype(F32) * 4, (rng.standard_normal(5000) * 1e3).astype(F32)])
+    if not os.path.exists(p):
+        want = json.load(open(stored))
+        for fmt in range(9):
+            assert _digest(o.convert_to_exmy(x, fmt)) == want[str(fmt)], fmt
+        return
+    h = ctypes.CDLL(p)
+    h.ref_convert_to_exmy_n.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_long, ctypes.c_int]
+    digests = {}
     for fmt in range(9):
         y = np.empty_like(x)
         h.ref_convert_to_exmy_n(x.ctypes.data, y.ctypes.data, x.size, fmt)
         assert same(o.convert_to_exmy(x, fmt), y).all()
+        digests[str(fmt)] = _digest(y)
+    if os.environ.get("B200Q_RECORD_GOLDEN"):
+        os.makedirs(os.environ["B200Q_RECORD_GOLDEN"], exist_ok=True)
+        with open(os.path.join(os.environ["B200Q_RECORD_GOLDEN"], "ref_mx_cvt_sha256.json"), "w") as fh:
+            json.dump(digests, fh, indent=1)
